@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- query frames/sec of the GATsSPG 2D-3D matching forward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic input:
 ``--frames`` (32) query frames of ONE object, N2D=1024, N3D=7000, L=8, D=256
@@ -135,6 +135,24 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm), "source": "nvidia-smi -lms 20"}
 
 
+DUMP_SAMPLE = 1 << 21        # elements kept of a larger output (the confidence matrix has 229 M at the default shape)
+
+
+def dump_outputs(path, out):
+    """Write the tensors of one call's result dict as <path>/<name>.npy: floating outputs as float32, index outputs as float64
+    (exact).  An output of more than DUMP_SAMPLE elements is written as its values at a fixed sample of flat indices (drawn by
+    numpy RandomState(0), sorted, repeats dropped): the same for every run at the same shape, so that the files of two builds
+    compare element for element.  At most 2^21 elements per file: under 60 MB for the five outputs of match_frames."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        if not torch.is_tensor(t):
+            continue
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.unique(np.random.RandomState(0).randint(0, t.numel(), DUMP_SAMPLE, dtype=np.int64))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy().astype(np.float32 if t.is_floating_point() else np.float64))
+
+
 def cpu_threads():
     """Threads for the CPU arm: all logical CPUs up to 32.  (Measured on the GPU box, 2x Xeon 8562Y+,
     128 logical CPUs: torch's CPU backend is >10x SLOWER at 128 threads than at 32 on this op mix --
@@ -202,7 +220,10 @@ def run_reference(args, rank, world):
     for w in range(args.warmup):
         _oracle_one(oracle, P, hp, synthetic.make_frame(w, db, N2D)[0], db, leaves)
     for s in range(args.steps):
-        per_step.append(_oracle_one(oracle, P, hp, synthetic.make_frame(1000 + s, db, N2D)[0], db, leaves)[0])
+        dt, out = _oracle_one(oracle, P, hp, synthetic.make_frame(1000 + s, db, N2D)[0], db, leaves)
+        per_step.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     total = sum(per_step)
     fps = args.steps / total
     line = {
@@ -577,6 +598,8 @@ def main():
     ap.add_argument("--chunk", type=int, default=0, help="frames per GNN chunk (0 = library default)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra legs (latency_b1, config4, config5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as DIR/<name>.npy "
+                                                          "(rank 0; inputs are seeded: the same arguments give the same inputs)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -657,6 +680,8 @@ def main():
     total_ms = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
     model.check_range()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     check_frame = 0
     check_conf = out["conf_matrix"][check_frame].cpu()
     check_m0 = out["matches0"][check_frame].cpu()

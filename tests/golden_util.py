@@ -1,9 +1,11 @@
 """Load a golden fixture (tests/golden/*.npz, made by make_golden.py from the
 reference module) and regenerate its seeded inputs."""
+import contextlib
 import glob
 import os
 
 import numpy as np
+import torch
 
 from onepose_b200 import synthetic
 
@@ -11,6 +13,21 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 FORWARD_CASES = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN_DIR, "*.npz"))
                        if not os.path.basename(p).startswith(("empty", "mean_", "features3d", "dustbin", "pnp_", "superpoint")))
 RELEASED_CASES = [c for c in FORWARD_CASES if not c.startswith(("noself", "lintrans", "additional"))]
+# make_golden.py records the fixtures on this many torch CPU threads.  How torch's fp32 convolutions split their sums depends on
+# the thread count: on 32 or 128 threads the SuperPoint scores move by ~1e-6 (up to 20 ulp), so a CPU recomputation that is
+# held to a fixture at fp32 rounding runs on the same count.
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    """Run the enclosed CPU computation on the thread count the fixtures were recorded with."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(n)
 
 
 def load_case(name):

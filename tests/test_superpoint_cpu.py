@@ -13,7 +13,7 @@ import torch.nn.functional as F
 from oracle import superpoint_oracle as O
 from onepose_b200 import SuperPoint, _lib, synthetic
 from tests import sp_emulation as E
-from tests.golden_util import GOLDEN_DIR, SUPERPOINT_CASES, load_superpoint_case
+from tests.golden_util import GOLDEN_DIR, SUPERPOINT_CASES, golden_threads, load_superpoint_case
 
 
 @pytest.mark.parametrize("name", SUPERPOINT_CASES)
@@ -22,7 +22,8 @@ def test_oracle_matches_reference_module(name):
     p = O.params_from_numpy(sd)
     every = int(g["meta_every"])
     for ac, tag in ((False, "ac0"), (True, "ac1")):
-        out = O.forward(p, img, conf, align_corners=ac)
+        with golden_threads():
+            out = O.forward(p, img, conf, align_corners=ac)
         for b in range(img.shape[0]):
             np.testing.assert_array_equal(out["keypoints"][b].numpy(), g[f"keypoints_{b}"])         # bit-exact key points
             np.testing.assert_allclose(out["scores"][b].numpy(), g[f"scores_{b}"], atol=1e-7)
