@@ -48,7 +48,7 @@ typedef struct opb_config {
 /* Replaces GATsSuperGlue.__init__ (GATs_SuperGlue.py:145-177). */
 int opb_create(const opb_config* cfg, opb_matcher** out);
 void opb_destroy(opb_matcher* m);
-const char* opb_last_error(const opb_matcher* m); /* m may be NULL: last create error */
+const char* opb_last_error(const opb_matcher* m); /* m may be NULL: message of this thread's last failed call that had no handle */
 
 /* Replaces nn.Module.load_state_dict for the keys of GATs_SuperGlue.py (SURVEY 2.1):
  * `name` is the reference state-dict key ("gnn.layers.1.attn.proj.0.weight", ...),
@@ -173,7 +173,7 @@ typedef struct opb_sp_config {
 
 int opb_sp_create(const opb_sp_config* cfg, opb_superpoint** out);
 void opb_sp_destroy(opb_superpoint* h);
-const char* opb_sp_last_error(const opb_superpoint* h); /* h may be NULL: last create error */
+const char* opb_sp_last_error(const opb_superpoint* h); /* h may be NULL: message of this thread's last failed call that had no handle */
 /* Reference state-dict keys ("conv1a.weight", "conv1a.bias", ... "convDb.bias"; superpoint.py:111-126), HOST fp32 arrays in
  * the reference's own [C_out, C_in, kh, kw] layout.  opb_sp_finalize_weights packs them (tap-major reduction index, the two
  * heads' 3x3 layers side by side, fp16 hi/lo split) and uploads. */

@@ -2,7 +2,6 @@
 // Host-side state: packed weights, per-object constants, chunk workspace, launch sequence.
 #include <algorithm>
 #include <cmath>
-#include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -23,7 +22,6 @@ namespace opb {
 constexpr int kDefaultChunk = 32;   // frames pushed through the GNN together (measured: 4 -> 1340, 8 -> 1650, 16 -> 2390, 32 -> 2550 frames/s)
 constexpr int kQPassFrames = 16;    // granularity of the query-side layer-1 pass when the queries stream in from the host
 
-static thread_local std::string g_create_error;
 static bool g_pdl = true;
 static int g_ws_fill = -1;     // >= 0: byte value written into every fresh allocation that the algorithm does not require to be zero
 int ws_fill_byte() { return g_ws_fill; }
@@ -44,10 +42,8 @@ struct AttnLayerW {       // one AttentionPropagation (reference GATs_SuperGlue.
 
 using namespace opb;
 
-struct opb_matcher {
+struct opb_matcher : HostState {
   opb_config cfg{};
-  std::string err;
-  std::map<std::string, std::vector<float>> host_w;
   bool weights_ready = false;
   bool object_ready = false;
   int num_sms = 148;
@@ -85,102 +81,18 @@ struct opb_matcher {
   std::vector<cudaEvent_t> h2d_ev;              // one per piece; consumed by the chunk loop of opb_forward
   int h2d_pending = 0;
   Layout last_layout{};
-  // profiling (bench.py roofline leg)
-  bool profiling = false;
-  std::vector<cudaEvent_t> ev_pool;
-  size_t ev_used = 0;
-  std::vector<double> ev_flops;     // per profiled launch (0 for the helper kernels)
-  std::vector<std::string> ev_name; // per profiled launch; an event is recorded AFTER every launch, durations = consecutive differences
-  cudaEvent_t ev_fwd0 = nullptr, ev_fwd1 = nullptr;
-  int launches = 0;
   int last_launches = 0;
 };
 
 namespace opb {
 
-int fail(opb_matcher* m, int code, const char* fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof buf, fmt, ap);
-  va_end(ap);
-  if (m) m->err = buf; else g_create_error = buf;
-  return code;
+// Profile name of a GEMM launch: "gemm epi<epilogue> n<N> k<K> <what>" (bench.py selects launches by its prefix), formatted
+// only when profiling.
+static int matcher_gemm(opb_matcher* m, const GemmProblem& p, cudaStream_t st, double flops, const char* what) {
+  char tag[96];
+  if (m->profiling) snprintf(tag, sizeof tag, "gemm epi%d n%d k%d %s", p.epi, p.n_out, p.K1 + p.K2, what);
+  return run_gemm(m, p, st, flops, m->profiling ? tag : what);
 }
-
-#define CK(m, expr)                                                                                   \
-  do {                                                                                                \
-    cudaError_t _e = (expr);                                                                          \
-    if (_e != cudaSuccess)                                                                            \
-      return fail(m, OPB_E_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
-  } while (0)
-
-// weight uploads are synchronous copies on the legacy stream; opb_finalize_weights ends with a device synchronisation so that
-// they are ordered against whatever (non-blocking) stream the caller uses afterwards
-static int upload_planes(opb_matcher* m, PlaneBuf& dst, const std::vector<double>& w, size_t off_elems = 0, size_t total_elems = 0) {
-  std::vector<__half> hi, lo;
-  split_host(w, hi, lo);
-  CK(m, dst.ensure(total_elems ? total_elems : w.size()));
-  CK(m, cudaMemcpy(dst.hi.as<__half>() + off_elems, hi.data(), hi.size() * sizeof(__half), cudaMemcpyHostToDevice));
-  CK(m, cudaMemcpy(dst.lo.as<__half>() + off_elems, lo.data(), lo.size() * sizeof(__half), cudaMemcpyHostToDevice));
-  return 0;
-}
-static int upload_f32(opb_matcher* m, DevBuf& dst, const std::vector<double>& w) {
-  std::vector<float> f(w.begin(), w.end());
-  CK(m, dst.ensure(f.size() * sizeof(float)));
-  CK(m, cudaMemcpy(dst.p, f.data(), f.size() * sizeof(float), cudaMemcpyHostToDevice));
-  return 0;
-}
-
-static const std::vector<float>* find_w(opb_matcher* m, const std::string& key, size_t n) {
-  auto it = m->host_w.find(key);
-  if (it == m->host_w.end()) { fail(m, OPB_E_STATE, "missing weight '%s'", key.c_str()); return nullptr; }
-  if (it->second.size() != n) {
-    fail(m, OPB_E_INVALID, "weight '%s' has %zu elements, expected %zu", key.c_str(), it->second.size(), n);
-    return nullptr;
-  }
-  return &it->second;
-}
-
-static cudaEvent_t next_event(opb_matcher* m) {
-  if (m->ev_used == m->ev_pool.size()) {
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    m->ev_pool.push_back(e);
-  }
-  return m->ev_pool[m->ev_used++];
-}
-
-// Profiling (bench.py roofline leg): one event after every launch on the stream; a launch's time is the difference to the
-// previous event (so it includes any launch gap in front of it).
-static void prof_mark(opb_matcher* m, cudaStream_t st, const char* name, double flops) {
-  if (!m->profiling) return;
-  cudaEventRecord(next_event(m), st);
-  m->ev_flops.push_back(flops);
-  m->ev_name.push_back(name);
-}
-
-// One launch of the tcgen05 GEMM core.  `flops` = algorithmic FLOPs.
-static int run_gemm(opb_matcher* m, const GemmProblem& p, cudaStream_t st, double flops, const char* what) {
-  const int rc = launch_gemm_tc(p, st);
-  if (m->profiling) {
-    char tag[96];
-    snprintf(tag, sizeof tag, "gemm epi%d n%d k%d %s", p.epi, p.n_out, p.K1 + p.K2, what);
-    prof_mark(m, st, tag, flops);
-  }
-  m->launches++;
-  if (rc != 0) return fail(m, rc == -1 ? OPB_E_INVALID : OPB_E_CUDA, "GEMM launch failed (%s, rc=%d): %s", what, rc,
-                           cudaGetErrorString(cudaGetLastError()));
-  return 0;
-}
-
-#define LAUNCH(m, st, name, ...)                                                                                    \
-  do {                                                                                                              \
-    cudaError_t _le = launch_k(__VA_ARGS__);                                                                        \
-    if (_le != cudaSuccess) return fail(m, OPB_E_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(_le));    \
-    (m)->launches++;                                                                                                \
-    prof_mark(m, st, name, 0.0);                                                                                    \
-  } while (0)
 
 static int ensure_workspace(opb_matcher* m, int frames, int N) {
   if (frames <= m->ws_frames && N <= m->ws_N) return 0;
@@ -246,7 +158,7 @@ static int run_gats(opb_matcher* m, const Layout& L, XView x, int gi, cudaStream
   p.L = Lc; p.batch = 1; p.rows = Lc.rows();
   p.a1 = m->lin_a.c(kD); p.K1 = kD; p.b1 = m->wlin.c(kD, (size_t)gi * kD * kD); p.n_out = kD;
   p.epi = EPI_BIAS_PLANES; p.out = m->lin_b.m(kD);
-  if (int rc = run_gemm(m, p, st, 2.0 * L.B * (double)L.M * kD * kD, "gats.W")) return rc;
+  if (int rc = matcher_gemm(m, p, st, 2.0 * L.B * (double)L.M * kD * kD, "gats.W")) return rc;
   const long long n = (long long)L.B * L.M * 32;
   LAUNCH(m, st, "gats_lin_finish", gats_lin_finish, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, st, (const __half*)m->lin_b.hi.as<__half>(),
          (const __half*)m->lin_b.lo.as<__half>(), x.hi, x.lo, L, (int)(m->cfg.include_self && m->cfg.additional));
@@ -267,12 +179,11 @@ static int run_attn_layer(opb_matcher* m, const Layout& L, XView x, AttnLayerW& 
   pk.bias = W.bqkv.as<float>() + 256;
   pk.epi = EPI_QKV; pk.out = Planes{m->kvt.as<__half>(), m->kvt.as<__half>(), 512};
   pk.a_hi_only = m->kv_two_pass;
-  if (int rc = run_gemm(m, pk, st, 2.0 * valid_rows * 512 * kD, "kv_proj")) return rc;
+  if (int rc = matcher_gemm(m, pk, st, 2.0 * valid_rows * 512 * kD, "kv_proj")) return rc;
   // (2) linear-attention state of every segment (:71-78): per-row-group partial states on the tensor cores ...
   const KvGroups G = kv_groups_for(L, m->num_sms);
   if (launch_kv_state_h(m->kvt.as<__half>(), L, G, m->kvpart.as<float>(), st)) return fail(m, OPB_E_CUDA, "kv_state_h launch failed");
-  m->launches++;
-  prof_mark(m, st, "kv_state_h", 0.0);
+  log_launch(m, st, "kv_state_h", 0.0);
   // ... reduced per segment into Kmean and the block-diagonal operand of the G fold (indexed by DESTINATION segment)
   LAUNCH(m, st, "kv_state_reduce", kv_state_reduce, dim3(S * kHeads, (kKVPartial + 255) / 256), dim3(256), 0, st, (const float*)m->kvpart.as<float>(), L,
          G, cross, m->kmean.as<float>(), m->bd.hi.as<__half>(), m->bd.lo.as<__half>());
@@ -281,7 +192,7 @@ static int run_attn_layer(opb_matcher* m, const Layout& L, XView x, AttnLayerW& 
   pq.L = L; pq.batch = 1; pq.rows = rows;
   pq.a1 = x.c(kD); pq.K1 = kD; pq.b1 = W.wqkv.c(kD); pq.n_out = 256; pq.bias = W.bqkv.as<float>();
   pq.epi = EPI_QSCALE; pq.kmean = m->kmean.as<float>(); pq.cross = cross; pq.out = m->qp.m(kD);
-  if (int rc = run_gemm(m, pq, st, 2.0 * valid_rows * 256 * kD, "q_proj")) return rc;
+  if (int rc = matcher_gemm(m, pq, st, 2.0 * valid_rows * 256 * kD, "q_proj")) return rc;
   // (4) dynamic weight G[s] = W0m . blockdiag(KVmean_src(s))^T  -- merge and the message half of mlp.0 folded into one
   //     per-segment [512, 256] weight (4 x 64x64x512 MACs per segment), as a batched tcgen05 GEMM over the segments
   GemmProblem pg{};
@@ -289,7 +200,7 @@ static int run_attn_layer(opb_matcher* m, const Layout& L, XView x, AttnLayerW& 
   pg.a1 = W.w0m.c(kD); pg.a_batch_rows = 0;
   pg.b1 = m->bd.c(kD); pg.b_batch_rows = kD;
   pg.epi = EPI_BIAS_PLANES; pg.out = m->g.m(kD);
-  if (int rc = run_gemm(m, pg, st, 2.0 * S * 512.0 * kD * kDh, "g_fold")) return rc;
+  if (int rc = matcher_gemm(m, pg, st, 2.0 * S * 512.0 * kD * kDh, "g_fold")) return rc;
   // (5) hidden = mlp.0([x ; message]) = [x | Q'] . [W0a | G_seg]^T + b   (:101,:113,:122); epilogue also emits the InstanceNorm
   //     partial sums (:126)
   GemmProblem p2{};
@@ -298,7 +209,7 @@ static int run_attn_layer(opb_matcher* m, const Layout& L, XView x, AttnLayerW& 
   p2.a2 = m->qp.c(kD); p2.K2 = kD; p2.b2 = m->g.c(kD); p2.b2_per_seg = 1;
   p2.n_out = 512; p2.bias = W.b0f.as<float>(); p2.c = m->hid.as<float>(); p2.ldc = 512;
   p2.epi = EPI_F32_STATS; p2.statpart = m->statpart.as<float>();
-  if (int rc = run_gemm(m, p2, st, 2.0 * valid_rows * 512 * 512, "mlp0")) return rc;
+  if (int rc = matcher_gemm(m, p2, st, 2.0 * valid_rows * 512 * 512, "mlp0")) return rc;
   // (6) InstanceNorm statistics per segment (:126)
   LAUNCH(m, st, "in_stats_final", in_stats_final, dim3(S, 16), dim3(32, kStatSlices), 0, st, (const float*)m->statpart.as<float>(), L, m->mu.as<float>(),
          m->rstd.as<float>());
@@ -309,7 +220,7 @@ static int run_attn_layer(opb_matcher* m, const Layout& L, XView x, AttnLayerW& 
   p3.epi = EPI_BIAS_PLANES; p3.out = x.m(kD);
   p3.a2 = x.c(kD); p3.K2 = kD; p3.b2 = m->eye.c(kD); p3.b2_lo_zero = 1; p3.b2_identity = m->identity_diag;
   p3.a_conv = 1; p3.a_raw = m->hid.as<float>(); p3.a_raw_ld = 512; p3.mu = m->mu.as<float>(); p3.rstd = m->rstd.as<float>();
-  return run_gemm(m, p3, st, 2.0 * valid_rows * 256 * 512, "mlp3");
+  return matcher_gemm(m, p3, st, 2.0 * valid_rows * 256 * 512, "mlp3");
 }
 
 // Object prologue: GNN layers 0 (GATs) and the 3D side of layer 1 (self-attention) depend only on the per-object
@@ -383,7 +294,7 @@ static int forward_chunk(opb_matcher* m, const float* q_cf, const int* nlen, int
   pf.a1 = m->x.c(kD); pf.K1 = kD; pf.b1 = m->wf.c(kD); pf.n_out = 256;
   pf.bias = m->bf.as<float>();
   pf.epi = EPI_L2NORM; pf.out = m->pn.m(kD);       // F.normalize fused into the final_proj epilogue (:209-213)
-  if (int rc = run_gemm(m, pf, st, 2.0 * valid_rows * kD * kD, "final_proj")) return rc;
+  if (int rc = matcher_gemm(m, pf, st, 2.0 * valid_rows * kD * kD, "final_proj")) return rc;
   // dual softmax + arg-max as two passes of the batched score GEMM (one batch = one frame); the cos matrix is never stored
   const int n_parts = (L.m_pad / 256) * 2, q_groups = L.n_pad / 32;
   GemmProblem ps{};
@@ -392,13 +303,13 @@ static int forward_chunk(opb_matcher* m, const float* q_cf, const int* nlen, int
   ps.a_batch_rows = L.R; ps.b_batch_rows = L.R;
   ps.inv_scale = 1.f / m->cfg.scale_factor;
   ps.epi = EPI_SCORE_SUMS; ps.rowsum_part = m->rowsum_part.as<float>(); ps.colsum_part = m->colsum_part.as<float>();
-  if (int rc = run_gemm(m, ps, st, 2.0 * fb * (double)N * L.M * kD, "score_sums")) return rc;
+  if (int rc = matcher_gemm(m, ps, st, 2.0 * fb * (double)N * L.M * kD, "score_sums")) return rc;
   LAUNCH(m, st, "score_sums_finalize", score_sums_finalize, dim3((L.n_pad + L.m_pad + 255) / 256, fb), dim3(256), 0, st,
          (const float*)m->rowsum_part.as<float>(), (const float*)m->colsum_part.as<float>(), L, n_parts, q_groups, m->rowsum.as<float>(),
          m->colsum.as<float>(), m->rowbest.as<unsigned long long>(), m->colbest.as<unsigned long long>());
   ps.epi = EPI_SCORE_CONF; ps.inv_rowsum = m->rowsum.as<float>(); ps.inv_colsum = m->colsum.as<float>();
   ps.conf = conf; ps.rowbest = m->rowbest.as<unsigned long long>(); ps.colbest = m->colbest.as<unsigned long long>();
-  if (int rc = run_gemm(m, ps, st, 0.0, "score_conf")) return rc;      // recomputation: its FLOPs are not algorithmic
+  if (int rc = matcher_gemm(m, ps, st, 0.0, "score_conf")) return rc;      // recomputation: its FLOPs are not algorithmic
   LAUNCH(m, st, "mutual_match", mutual_match, dim3(fb), dim3(256), 0, st, (const unsigned long long*)m->rowbest.as<unsigned long long>(),
          (const unsigned long long*)m->colbest.as<unsigned long long>(), L, m->cfg.match_threshold, (const int*)m->range_flag.as<int>(),
          reinterpret_cast<long long*>(m0), reinterpret_cast<long long*>(m1), s0, s1);
@@ -432,6 +343,7 @@ int opb_create(const opb_config* cfg, opb_matcher** out) {
   if (prop.major != 10) return fail(nullptr, OPB_E_CUDA, "device is sm_%d%d; this library is built for sm_100a only", prop.major, prop.minor);
   auto* m = new opb_matcher();
   m->cfg = *cfg;
+  m->device = cfg->device;
   m->num_sms = prop.multiProcessorCount;
   if (cudaMallocHost(&m->range_host, sizeof(int)) != cudaSuccess || cudaEventCreateWithFlags(&m->range_ev, cudaEventDisableTiming) != cudaSuccess) {
     delete m;
@@ -444,7 +356,7 @@ int opb_create(const opb_config* cfg, opb_matcher** out) {
 
 void opb_destroy(opb_matcher* m) {
   if (!m) return;
-  cudaSetDevice(m->cfg.device);
+  cudaSetDevice(m->device);
   cudaDeviceSynchronize();
   for (auto& a : m->attn) { a.wqkv.release(); a.bqkv.release(); a.w0a.release(); a.w0m.release(); a.b0f.release(); a.w1.release(); a.b1.release(); }
   DevBuf* bufs[] = {&m->wa2, &m->wa3, &m->bf, &m->leaves, &m->s2, &m->kvt, &m->hid, &m->kvpart, &m->kmean, &m->statpart,
@@ -453,27 +365,25 @@ void opb_destroy(opb_matcher* m) {
   for (auto* b : bufs) b->release();
   PlaneBuf* pb[] = {&m->wf, &m->wlin, &m->db, &m->xo, &m->x, &m->qp, &m->pn, &m->g, &m->xq, &m->bd, &m->lin_a, &m->lin_b, &m->eye};
   for (auto* b : pb) b->release();
-  for (auto e : m->ev_pool) cudaEventDestroy(e);
   for (auto e : m->h2d_ev) cudaEventDestroy(e);
   if (m->copy_stream) cudaStreamDestroy(m->copy_stream);
-  if (m->ev_fwd0) { cudaEventDestroy(m->ev_fwd0); cudaEventDestroy(m->ev_fwd1); }
   if (m->range_ev) cudaEventDestroy(m->range_ev);
   if (m->range_host) cudaFreeHost(m->range_host);
   delete m;
 }
 
-const char* opb_last_error(const opb_matcher* m) { return m ? m->err.c_str() : g_create_error.c_str(); }
+const char* opb_last_error(const opb_matcher* m) { return m ? m->err.c_str() : g_last_error.c_str(); }
 
 int opb_load_weight(opb_matcher* m, const char* name, const float* data, size_t n) {
-  if (!m || !name || !data) return fail(m, OPB_E_INVALID, "null argument");
+  ENTER(m);
+  if (!name || !data) return fail(m, OPB_E_INVALID, "opb_load_weight: null argument");
   m->host_w[name] = std::vector<float>(data, data + n);
   m->weights_ready = false;
   return OPB_OK;
 }
 
 int opb_finalize_weights(opb_matcher* m) {
-  if (!m) return OPB_E_INVALID;
-  CK(m, cudaSetDevice(m->cfg.device));
+  ENTER(m);
   // head-contiguous channel order: new c' = h*64 + d  <-  reference c = d*4 + h (GATs_SuperGlue.py:97)
   int perm[kD];
   for (int h = 0; h < kHeads; ++h)
@@ -483,9 +393,9 @@ int opb_finalize_weights(opb_matcher* m) {
   for (int layer = 0; layer < 12; ++layer) {
     const std::string p = "gnn.layers." + std::to_string(layer);
     if (layer % 3 == 0) {
-      auto* W = find_w(m, p + ".W", kD * kD);
-      auto* a = find_w(m, p + ".a", 2 * kD);
-      if (!W || !a) return OPB_E_STATE;
+      const std::vector<float> *W, *a;
+      if (int rc = find_w(m, p + ".W", kD * kD, W)) return rc;
+      if (int rc = find_w(m, p + ".a", 2 * kD, a)) return rc;
       const int gi = layer / 3;
       for (int c = 0; c < kD; ++c) {  // h @ W @ a[:256] = h . (W a[:256])   (GATs.py:40,78-80)
         double s2 = 0, s3 = 0;
@@ -505,19 +415,17 @@ int opb_finalize_weights(opb_matcher* m) {
       continue;
     }
     AttnLayerW& A = m->attn[ai++];
-    const std::vector<float>*Wp[3], *bp[3];
+    const std::vector<float>*Wp[3], *bp[3], *Wm, *bm, *W0, *b0, *W1, *b1;
     for (int j = 0; j < 3; ++j) {
-      Wp[j] = find_w(m, p + ".attn.proj." + std::to_string(j) + ".weight", kD * kD);
-      bp[j] = find_w(m, p + ".attn.proj." + std::to_string(j) + ".bias", kD);
-      if (!Wp[j] || !bp[j]) return OPB_E_STATE;
+      if (int rc = find_w(m, p + ".attn.proj." + std::to_string(j) + ".weight", kD * kD, Wp[j])) return rc;
+      if (int rc = find_w(m, p + ".attn.proj." + std::to_string(j) + ".bias", kD, bp[j])) return rc;
     }
-    auto* Wm = find_w(m, p + ".attn.merge.weight", kD * kD);
-    auto* bm = find_w(m, p + ".attn.merge.bias", kD);
-    auto* W0 = find_w(m, p + ".mlp.0.weight", 512 * 512);
-    auto* b0 = find_w(m, p + ".mlp.0.bias", 512);
-    auto* W1 = find_w(m, p + ".mlp.3.weight", kD * 512);
-    auto* b1 = find_w(m, p + ".mlp.3.bias", kD);
-    if (!Wm || !bm || !W0 || !b0 || !W1 || !b1) return OPB_E_STATE;
+    if (int rc = find_w(m, p + ".attn.merge.weight", kD * kD, Wm)) return rc;
+    if (int rc = find_w(m, p + ".attn.merge.bias", kD, bm)) return rc;
+    if (int rc = find_w(m, p + ".mlp.0.weight", 512 * 512, W0)) return rc;
+    if (int rc = find_w(m, p + ".mlp.0.bias", 512, b0)) return rc;
+    if (int rc = find_w(m, p + ".mlp.3.weight", kD * 512, W1)) return rc;
+    if (int rc = find_w(m, p + ".mlp.3.bias", kD, b1)) return rc;
     std::vector<double> wqkv(768 * kD), bqkv(768);
     for (int j = 0; j < 3; ++j)
       for (int c = 0; c < kD; ++c) {
@@ -536,25 +444,24 @@ int opb_finalize_weights(opb_matcher* m) {
         w0m[(size_t)c * kD + k] = acc;
       }
     }
-    std::vector<double> w1(W1->begin(), W1->end()), b1d(b1->begin(), b1->end());
     if (int rc = upload_planes(m, A.wqkv, wqkv)) return rc;
     if (int rc = upload_f32(m, A.bqkv, bqkv)) return rc;
     if (int rc = upload_planes(m, A.w0a, w0a)) return rc;
     if (int rc = upload_planes(m, A.w0m, w0m)) return rc;
     if (int rc = upload_f32(m, A.b0f, b0f)) return rc;
-    if (int rc = upload_planes(m, A.w1, w1)) return rc;
-    if (int rc = upload_f32(m, A.b1, b1d)) return rc;
+    if (int rc = upload_planes(m, A.w1, std::vector<double>(W1->begin(), W1->end()))) return rc;
+    if (int rc = upload_f32(m, A.b1, *b1)) return rc;
   }
-  auto* Wf = find_w(m, "final_proj.weight", kD * kD);
-  auto* bfv = find_w(m, "final_proj.bias", kD);
-  if (!Wf || !bfv) return OPB_E_STATE;
+  const std::vector<float> *Wf, *bfv;
+  if (int rc = find_w(m, "final_proj.weight", kD * kD, Wf)) return rc;
+  if (int rc = find_w(m, "final_proj.bias", kD, bfv)) return rc;
   if (int rc = upload_planes(m, m->wf, std::vector<double>(Wf->begin(), Wf->end()))) return rc;
   {
     std::vector<double> eye((size_t)kD * kD, 0.0);
     for (int i = 0; i < kD; ++i) eye[(size_t)i * kD + i] = 1.0;
     if (int rc = upload_planes(m, m->eye, eye)) return rc;
   }
-  if (int rc = upload_f32(m, m->bf, std::vector<double>(bfv->begin(), bfv->end()))) return rc;
+  if (int rc = upload_f32(m, m->bf, *bfv)) return rc;
   if (int rc = upload_f32(m, m->wa2, wa2)) return rc;
   if (int rc = upload_f32(m, m->wa3, wa3)) return rc;
   CK(m, cudaDeviceSynchronize());
@@ -565,11 +472,10 @@ int opb_finalize_weights(opb_matcher* m) {
 }
 
 int opb_set_object(opb_matcher* m, const float* desc3d_db, const float* desc2d_db, int32_t M, int32_t Lf, void* stream) {
-  if (!m) return OPB_E_INVALID;
+  ENTER(m);
   if (!m->weights_ready) return fail(m, OPB_E_STATE, "opb_set_object before opb_finalize_weights");
   if (!desc3d_db || !desc2d_db || M <= 0 || Lf <= 0 || Lf > 32)
     return fail(m, OPB_E_INVALID, "set_object: need M > 0 and 1 <= num_leaf <= 32 (got M=%d, L=%d)", M, Lf);
-  CK(m, cudaSetDevice(m->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const int m_pad = round_up(M, kSegPad);
   if (m_pad != m->m_pad) { m->ws_frames = 0; m->ws_N = 0; }  // workspace depends on m_pad
@@ -595,41 +501,34 @@ int opb_set_object(opb_matcher* m, const float* desc3d_db, const float* desc2d_d
 }
 
 int opb_reserve_workspace(opb_matcher* m, int32_t frames, int32_t N) {
-  if (!m || frames <= 0 || N <= 0) return OPB_E_INVALID;
+  ENTER(m);
+  if (frames <= 0 || N <= 0) return fail(m, OPB_E_INVALID, "opb_reserve_workspace: bad argument (frames=%d, N=%d)", frames, N);
   if (!m->object_ready) return fail(m, OPB_E_STATE, "opb_reserve_workspace needs an object (the workspace depends on M)");
-  CK(m, cudaSetDevice(m->cfg.device));
   return ensure_workspace(m, chunk_of(m, frames), N);
 }
 
 int opb_set_hoist(opb_matcher* m, int32_t enable) {
-  if (!m) return OPB_E_INVALID;
+  ENTER(m);
   m->hoist = enable != 0;
   return OPB_OK;
 }
 
 int opb_set_chunk_frames(opb_matcher* m, int32_t frames) {
-  if (!m || frames < 0) return OPB_E_INVALID;
+  ENTER(m);
+  if (frames < 0) return fail(m, OPB_E_INVALID, "opb_set_chunk_frames: frames %d < 0", frames);
   m->chunk_frames = frames;
   return OPB_OK;
 }
 
 int opb_forward(opb_matcher* m, const float* q, const int32_t* n2d_lengths, int32_t B, int32_t N, int64_t* m0, int64_t* m1, float* s0, float* s1,
                 float* conf, void* stream) {
-  if (!m) return OPB_E_INVALID;
+  ENTER(m);
   if (!m->weights_ready || !m->object_ready) return fail(m, OPB_E_STATE, "opb_forward needs weights and an object (finalize_weights, set_object)");
   if (!q || !m0 || !m1 || !s0 || !s1 || B <= 0 || N <= 0) return fail(m, OPB_E_INVALID, "opb_forward: bad argument (B=%d, N=%d)", B, N);
-  CK(m, cudaSetDevice(m->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const int chunk = chunk_of(m, B);
   if (int rc = ensure_workspace(m, chunk, N)) return rc;   // no-op once opb_reserve_workspace / an earlier call has sized it
-  m->launches = 0;
-  if (m->profiling) {
-    m->ev_used = 0;
-    m->ev_flops.clear();
-    m->ev_name.clear();
-    if (!m->ev_fwd0) { cudaEventCreate(&m->ev_fwd0); cudaEventCreate(&m->ev_fwd1); }
-    cudaEventRecord(m->ev_fwd0, st);
-  }
+  begin_call(m, st);
   if (m->hoist && !m->prologue_ready) {
     if (int rc = object_prologue(m, st)) return rc;
     m->prologue_ready = true;
@@ -651,35 +550,34 @@ int opb_forward(opb_matcher* m, const float* q, const int32_t* n2d_lengths, int3
   CK(m, cudaEventRecord(m->range_ev, st));
   m->range_pending = true;
   m->last_stream = st;
-  if (m->profiling) cudaEventRecord(m->ev_fwd1, st);
+  end_call(m, st);
   m->last_launches = m->launches;
   return OPB_OK;
 }
 
 int opb_set_profiling(opb_matcher* m, int32_t enable) {
-  if (!m) return OPB_E_INVALID;
+  ENTER(m);
   m->profiling = enable != 0;
-  m->ev_used = 0;
-  m->ev_flops.clear();
-  m->ev_name.clear();
   return OPB_OK;
 }
 
 int opb_get_profile(opb_matcher* m, double* gemm_ms, double* gemm_flops, int32_t* gemm_launches, double* total_ms) {
-  if (!m || !m->ev_fwd1) return OPB_E_STATE;
-  CK(m, cudaEventSynchronize(m->ev_fwd1));
+  if (!m) return fail(nullptr, OPB_E_STATE, "opb_get_profile: null handle");
+  ENTER(m);
+  if (!m->ev_end) return fail(m, OPB_E_STATE, "opb_get_profile: no profiled call");
+  CK(m, cudaEventSynchronize(m->ev_end));
   double ms = 0, fl = 0;
   int n_gemm = 0;
   std::map<std::string, std::pair<double, std::pair<double, int>>> agg;
   for (size_t i = 0; i < m->ev_flops.size(); ++i) {
     float t = 0;
-    CK(m, cudaEventElapsedTime(&t, i == 0 ? m->ev_fwd0 : m->ev_pool[i - 1], m->ev_pool[i]));
+    if (int rc = entry_ms(m, i, &t)) return rc;
     if (m->ev_name[i].compare(0, 4, "gemm") == 0) { ms += t; fl += m->ev_flops[i]; ++n_gemm; }
     auto& a = agg[m->ev_name[i]];
     a.first += t; a.second.first += m->ev_flops[i]; a.second.second++;
   }
   float tot = 0;
-  CK(m, cudaEventElapsedTime(&tot, m->ev_fwd0, m->ev_fwd1));
+  CK(m, cudaEventElapsedTime(&tot, m->ev[0], m->ev_end));
   if (getenv("OPB_PROFILE_DUMP")) {   // measurement aid only: prints the table, selects nothing
     fprintf(stderr, "[opb profile] forward %.3f ms, GEMM %.3f ms in %d launches\n", tot, ms, n_gemm);
     for (auto& kv : agg)
@@ -694,15 +592,17 @@ int opb_get_profile(opb_matcher* m, double* gemm_ms, double* gemm_flops, int32_t
 }
 
 int opb_get_profile_entry(opb_matcher* m, const char* prefix, double* ms_out, double* flops_out, int32_t* launches_out) {
-  if (!m || !prefix || !m->ev_fwd1) return OPB_E_STATE;
-  CK(m, cudaEventSynchronize(m->ev_fwd1));
+  if (!m) return fail(nullptr, OPB_E_STATE, "opb_get_profile_entry: null handle");
+  ENTER(m);
+  if (!prefix || !m->ev_end) return fail(m, OPB_E_STATE, "opb_get_profile_entry: no prefix or no profiled call");
+  CK(m, cudaEventSynchronize(m->ev_end));
   double ms = 0, fl = 0;
   int n = 0;
   const size_t pl = strlen(prefix);
   for (size_t i = 0; i < m->ev_flops.size(); ++i) {
     if (m->ev_name[i].compare(0, pl, prefix) != 0) continue;
     float t = 0;
-    CK(m, cudaEventElapsedTime(&t, i == 0 ? m->ev_fwd0 : m->ev_pool[i - 1], m->ev_pool[i]));
+    if (int rc = entry_ms(m, i, &t)) return rc;
     ms += t; fl += m->ev_flops[i]; ++n;
   }
   if (ms_out) *ms_out = ms;
@@ -713,10 +613,9 @@ int opb_get_profile_entry(opb_matcher* m, const char* prefix, double* ms_out, do
 
 int opb_forward_host(opb_matcher* m, const float* qh, const int32_t* n2d_lengths_host, int32_t B, int32_t N, int64_t* m0h, int64_t* m1h, float* s0h,
                      float* s1h, float* confh, int32_t materialize_conf, void* stream) {
-  if (!m) return OPB_E_INVALID;
+  ENTER(m);
   if (!m->object_ready) return fail(m, OPB_E_STATE, "opb_forward_host needs an object");
   if (!qh || !m0h || !m1h || !s0h || !s1h || B <= 0 || N <= 0) return fail(m, OPB_E_INVALID, "opb_forward_host: bad argument");
-  CK(m, cudaSetDevice(m->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const size_t M = m->M;
   const bool want_conf = confh != nullptr || materialize_conf != 0;
@@ -782,12 +681,14 @@ static int consume_range_flag(opb_matcher* m) {
 int opb_check_range(opb_matcher* m, void* stream) {
   if (!m || !m->range_flag.p || !m->range_pending) return OPB_OK;
   (void)stream;
+  CK(m, cudaSetDevice(m->device));
   CK(m, cudaEventSynchronize(m->range_ev));
   return consume_range_flag(m);
 }
 
 int opb_poll_range(opb_matcher* m) {
   if (!m || !m->range_pending) return OPB_OK;
+  CK(m, cudaSetDevice(m->device));
   const cudaError_t q = cudaEventQuery(m->range_ev);
   if (q == cudaErrorNotReady) return OPB_OK;               // the call is still running: report on a later poll / check
   if (q != cudaSuccess) return fail(m, OPB_E_CUDA, "cudaEventQuery: %s", cudaGetErrorString(q));
@@ -797,54 +698,58 @@ int opb_poll_range(opb_matcher* m) {
 int opb_last_launch_count(const opb_matcher* m) { return m ? m->last_launches : 0; }
 
 // ---- adjacent producers ------------------------------------------------------------------
-static int scan_offsets(const int64_t* seg_len, int32_t M, long long** offs, cudaStream_t st) {
-  if (cudaMallocAsync(offs, (size_t)M * sizeof(long long), st) != cudaSuccess) return OPB_E_CUDA;
+static int scan_offsets(const int64_t* seg_len, int32_t M, long long** offs, cudaStream_t st, const char* fn) {
+  const cudaError_t e = cudaMallocAsync(offs, (size_t)M * sizeof(long long), st);
+  if (e != cudaSuccess) return fail(nullptr, OPB_E_CUDA, "%s: cudaMallocAsync failed: %s", fn, cudaGetErrorString(e));
   exclusive_scan_i64<<<1, 1024, 0, st>>>(reinterpret_cast<const long long*>(seg_len), *offs, M);
   return OPB_OK;
 }
 
 int opb_segmented_mean_f64(const double* desc, const int64_t* seg_len, int32_t M, int32_t D, double* out, void* stream) {
-  if (!desc || !seg_len || !out || M <= 0 || D <= 0) return OPB_E_INVALID;
+  if (!desc || !seg_len || !out || M <= 0 || D <= 0) return fail(nullptr, OPB_E_INVALID, "%s: bad argument (M=%d, D=%d)", __func__, M, D);
   cudaStream_t st = (cudaStream_t)stream;
   long long* offs = nullptr;
-  if (int rc = scan_offsets(seg_len, M, &offs, st)) return rc;
+  if (int rc = scan_offsets(seg_len, M, &offs, st, __func__)) return rc;
   segmented_mean_f64<<<(unsigned)(((long long)M * 32 + 255) / 256), 256, 0, st>>>(desc, reinterpret_cast<const long long*>(seg_len), offs, M, D, out);
   cudaFreeAsync(offs, st);
-  return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+  return launch_status(nullptr, __func__);
 }
 
 int opb_segmented_mean_scores_f64(const double* scores, const int64_t* seg_len, int32_t M, double* out, void* stream) {
-  if (!scores || !seg_len || !out || M <= 0) return OPB_E_INVALID;
+  if (!scores || !seg_len || !out || M <= 0) return fail(nullptr, OPB_E_INVALID, "%s: bad argument (M=%d)", __func__, M);
   cudaStream_t st = (cudaStream_t)stream;
   long long* offs = nullptr;
-  if (int rc = scan_offsets(seg_len, M, &offs, st)) return rc;
+  if (int rc = scan_offsets(seg_len, M, &offs, st, __func__)) return rc;
   segmented_mean_scores_f64<<<(unsigned)((M + 127) / 128), 128, 0, st>>>(scores, reinterpret_cast<const long long*>(seg_len), offs, M, out);
   cudaFreeAsync(offs, st);
-  return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+  return launch_status(nullptr, __func__);
 }
 
 int opb_gather_features3d(const float* desc, const float* scores, int32_t dim, int64_t n_src, const int64_t* idx, int64_t n_idx, float* desc_out,
                           float* scores_out, int64_t n_out, void* stream) {
-  if (!desc || !desc_out || dim <= 0 || n_src < 0 || n_out <= 0 || n_idx < 0 || n_idx > n_out) return OPB_E_INVALID;
+  if (!desc || !desc_out || dim <= 0 || n_src < 0 || n_out <= 0 || n_idx < 0 || n_idx > n_out)
+    return fail(nullptr, OPB_E_INVALID, "%s: bad argument (dim=%d, n_src=%lld, n_idx=%lld, n_out=%lld)", __func__, dim, (long long)n_src,
+                (long long)n_idx, (long long)n_out);
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned gx = (unsigned)((n_out + 255) / 256);
   gather_columns_f32<<<dim3(gx, (unsigned)dim), 256, 0, st>>>(desc, dim, (long long)n_src, reinterpret_cast<const long long*>(idx), (long long)n_idx,
                                                               desc_out, (long long)n_out);
   if (scores && scores_out)
     gather_scores_f32<<<gx, 256, 0, st>>>(scores, (long long)n_src, reinterpret_cast<const long long*>(idx), (long long)n_idx, scores_out, (long long)n_out);
-  return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+  return launch_status(nullptr, __func__);
 }
 
 // ---- test hooks ---------------------------------------------------------------------------
 int opb_debug_set_kv_passes(opb_matcher* m, int32_t passes) {
-  if (!m || (passes != 2 && passes != 3)) return OPB_E_INVALID;
+  ENTER(m);
+  if (passes != 2 && passes != 3) return fail(m, OPB_E_INVALID, "opb_debug_set_kv_passes: passes %d is not 2 or 3", passes);
   m->kv_two_pass = passes == 2 ? 1 : 0;
   m->prologue_ready = false;
   return OPB_OK;
 }
 
 int opb_debug_set_identity_diag(opb_matcher* m, int32_t enable) {
-  if (!m) return OPB_E_INVALID;
+  ENTER(m);
   m->identity_diag = enable ? 1 : 0;
   m->prologue_ready = false;
   return OPB_OK;
@@ -860,6 +765,12 @@ int opb_debug_set_pdl(int32_t enable) {
   return OPB_OK;
 }
 
+// Status of a GEMM launch of a debug hook: launch_gemm_* return -1 for a rejected problem, -2 for a CUDA error.
+static int gemm_status(int rc, const char* fn) {
+  if (rc == 0) return OPB_OK;
+  return fail(nullptr, rc == -1 ? OPB_E_INVALID : OPB_E_CUDA, "%s: GEMM launch failed (rc=%d)", fn, rc);
+}
+
 static GemmProblem plain_problem(const void* a_hi, const void* a_lo, const void* b_hi, const void* b_lo, float* c, int32_t rows, int32_t n_out, int32_t K) {
   GemmProblem p{};
   p.a1 = CPlanes{(const __half*)a_hi, (const __half*)a_lo, K};
@@ -871,21 +782,19 @@ static GemmProblem plain_problem(const void* a_hi, const void* a_lo, const void*
 int opb_debug_gemm(const void* a_hi, const void* a_lo, const void* b_hi, const void* b_lo, float* c, int32_t rows, int32_t n_out, int32_t K,
                    int32_t backend, void* stream) {
   GemmProblem p = plain_problem(a_hi, a_lo, b_hi, b_lo, c, rows, n_out, K);
-  int rc = backend == 1 ? launch_gemm_simt(p, (cudaStream_t)stream) : launch_gemm_tc(p, (cudaStream_t)stream);
-  return rc == 0 ? OPB_OK : (rc == -1 ? OPB_E_INVALID : OPB_E_CUDA);
+  return gemm_status(backend == 1 ? launch_gemm_simt(p, (cudaStream_t)stream) : launch_gemm_tc(p, (cudaStream_t)stream), __func__);
 }
 
 int opb_debug_gemm_timeline(const void* a_hi, const void* a_lo, const void* b_hi, const void* b_lo, float* c, int32_t rows, int32_t n_out,
                             int32_t K, long long* timeline, void* stream) {
   GemmProblem p = plain_problem(a_hi, a_lo, b_hi, b_lo, c, rows, n_out, K);
-  int rc = launch_gemm_tc(p, (cudaStream_t)stream, timeline);
-  return rc == 0 ? OPB_OK : (rc == -1 ? OPB_E_INVALID : OPB_E_CUDA);
+  return gemm_status(launch_gemm_tc(p, (cudaStream_t)stream, timeline), __func__);
 }
 
 int opb_debug_gemm_aconv(const float* a_raw, const void* b_hi, const void* b_lo, void* x_hi, void* x_lo, const float* mu, const float* rstd,
                          const float* bias, const void* eye_hi, const void* eye_lo, int32_t rows, long long* timeline, void* stream) {
   // the mlp.3 problem of one segment: x[rows,256] = [ReLU((a_raw - mu) * rstd) | x] . [B | I]^T + bias, converters on
-  if (!eye_hi || !eye_lo) return OPB_E_INVALID;
+  if (!eye_hi || !eye_lo) return fail(nullptr, OPB_E_INVALID, "%s: null identity planes", __func__);
   GemmProblem p{};
   p.b1 = CPlanes{(const __half*)b_hi, (const __half*)b_lo, 512};
   p.K1 = 512; p.rows = rows; p.n_out = 256; p.batch = 1; p.bias = bias;
@@ -894,8 +803,7 @@ int opb_debug_gemm_aconv(const float* a_raw, const void* b_hi, const void* b_lo,
   p.a2 = CPlanes{(const __half*)x_hi, (const __half*)x_lo, kD}; p.K2 = kD; p.b2 = CPlanes{(const __half*)eye_hi, (const __half*)eye_lo, kD};
   p.b2_lo_zero = 1; p.b2_identity = 1;
   p.a_conv = 1; p.a_raw = a_raw; p.a_raw_ld = 512; p.mu = mu; p.rstd = rstd;
-  int rc = launch_gemm_tc(p, (cudaStream_t)stream, timeline);
-  return rc == 0 ? OPB_OK : (rc == -1 ? OPB_E_INVALID : OPB_E_CUDA);
+  return gemm_status(launch_gemm_tc(p, (cudaStream_t)stream, timeline), __func__);
 }
 
 int opb_debug_kv_state_h(const void* kvh, int32_t frames, int32_t n, int32_t m_pts, int32_t slabs_per_group, float* partial, int32_t* n_groups,
@@ -911,23 +819,25 @@ int opb_debug_kv_state_h(const void* kvh, int32_t frames, int32_t n, int32_t m_p
   }
   if (n_groups) *n_groups = frames * (G.gq + G.gd);
   if (!partial) return OPB_OK;                    // size query
-  return launch_kv_state_h((const __half*)kvh, L, G, partial, (cudaStream_t)stream) == 0 ? OPB_OK : OPB_E_CUDA;
+  if (launch_kv_state_h((const __half*)kvh, L, G, partial, (cudaStream_t)stream)) return fail(nullptr, OPB_E_CUDA, "%s: launch failed", __func__);
+  return OPB_OK;
 }
 
 int opb_debug_split(const float* x, void* hi, void* lo, size_t n, void* stream) {
   split_planes<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, (__half*)hi, (__half*)lo, (long long)n);
-  return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+  return launch_status(nullptr, __func__);
 }
 
 int opb_debug_read(opb_matcher* m, int32_t which, float* out, size_t cap, int64_t* rows, void* stream) {
-  if (!m || !out) return OPB_E_INVALID;
+  ENTER(m);
+  if (!out) return fail(m, OPB_E_INVALID, "debug_read: null output");
   const Layout& L = m->last_layout;
   if (which == 0) {
     size_t n = (size_t)L.rows() * kD;
     if (rows) *rows = L.rows();
     if (n > cap) return fail(m, OPB_E_INVALID, "debug_read: capacity %zu < %zu", cap, n);
     join_planes<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(m->x.hi.as<__half>(), m->x.lo.as<__half>(), out, (long long)n);
-    return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+    return launch_status(m, __func__);
   }
   return fail(m, OPB_E_INVALID, "debug_read: unknown buffer %d", which);
 }

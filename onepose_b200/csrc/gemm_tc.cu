@@ -28,6 +28,7 @@
 #include <tuple>
 
 #include "gemm_tc.cuh"
+#include "host_util.cuh"
 
 namespace opb {
 namespace {
@@ -1108,25 +1109,22 @@ bool make_map3(CUtensorMap* out, const float* ptr, int M, int N, int B) {
 int g_conv_halo = 1;      // 0: nine row-shifted boxes per tile; 1: halo boxes (default)
 int conv_halo_mode() { return g_conv_halo; }
 
+// SM count of the current device, cached per device.
 int num_sms() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-  }
-  return n;
+  static std::mutex mu;
+  static std::map<int, int> n;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  std::lock_guard<std::mutex> lock(mu);
+  int& sms = n[dev];
+  if (!sms) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  return sms;
 }
 
 template <int EPI, int ACV = ACV_NONE, bool HI = false, int BN_ = 256>
 cudaError_t launch_variant(const cudaLaunchConfig_t& cfg, const Maps& mp, const TcParams& tp) {
-  static bool attr_done = false;
   auto* kern = gemm_tc_kernel<EPI, ACV, HI, BN_>;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
+  if (cudaError_t e = ensure_smem_attr((const void*)kern, kSmemBytes)) return e;
   return cudaLaunchKernelEx(&cfg, kern, mp, tp);
 }
 
@@ -1211,7 +1209,8 @@ int launch_gemm_tc(const GemmProblem& p, cudaStream_t stream, long long* timelin
   tp.kmean = p.kmean; tp.cross = p.cross; tp.statpart = p.statpart;
   if ((p.epi == EPI_QSCALE || p.b2_per_seg || p.epi == EPI_QKV || p.epi == EPI_F32_STATS || p.a_conv) && !tp.seg_rows) return -1;
   const int total_units = (tp.m_tiles / 2) * tp.n_tiles * tp.batch;
-  const int grid = total_units * 2 < num_sms() ? total_units * 2 : (num_sms() / 2) * 2;
+  const int sms = num_sms();
+  const int grid = total_units * 2 < sms ? total_units * 2 : (sms / 2) * 2;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(threads_of(p.a_conv));

@@ -12,6 +12,7 @@
 
 #include "common.cuh"
 #include "gemm_tc.cuh"
+#include "host_util.cuh"
 #include "kv_state_tc.cuh"
 
 namespace opb {
@@ -252,11 +253,7 @@ KvGroups kv_groups_for(const Layout& L, int num_sms) {
 }
 
 int launch_kv_state_h(const __half* kvh, const Layout& L, const KvGroups& G, float* partial, cudaStream_t stream) {
-  static bool attr_done = false;
-  if (!attr_done) {
-    if (cudaFuncSetAttribute(kv_state_h_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHSmemBytes) != cudaSuccess) return -2;
-    attr_done = true;
-  }
+  if (ensure_smem_attr((const void*)kv_state_h_kernel, kHSmemBytes) != cudaSuccess) return -2;
   CUtensorMap map;
   if (!make_tensor_map_2d(&map, kvh, L.rows(), 512, 512, 64, kHRows, false)) return -2;
   cudaLaunchConfig_t cfg{};

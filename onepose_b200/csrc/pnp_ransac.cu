@@ -17,6 +17,7 @@
 #include <stdint.h>
 
 #include "../../include/onepose_b200.h"
+#include "host_util.cuh"
 
 namespace opb {
 namespace {
@@ -374,11 +375,11 @@ extern "C" int opb_ransac_pnp(const double* K, const double* pts2d, const double
                               double reproj_error, uint64_t seed, double* workspace, double* pose_out, int32_t* inlier_mask, int32_t* n_inliers,
                               void* stream) {
   if (!K || !pts2d || !pts3d || !offsets || !workspace || !pose_out || !inlier_mask || !n_inliers || B <= 0 || hypotheses <= 0 || !(reproj_error > 0.0))
-    return OPB_E_INVALID;
+    return opb::fail(nullptr, OPB_E_INVALID, "%s: bad argument (B=%d, hypotheses=%d, reproj_error=%g)", __func__, B, hypotheses, reproj_error);
   cudaStream_t st = (cudaStream_t)stream;
   const double thr2 = reproj_error * reproj_error;
   opb::pnp_hypotheses<<<dim3((unsigned)((hypotheses + 127) / 128), (unsigned)B), 128, 0, st>>>(K, pts2d, pts3d, offsets, hypotheses, thr2,
                                                                                                (unsigned long long)seed, workspace);
   opb::pnp_select_refine<<<(unsigned)B, opb::kRefineThreads, 0, st>>>(K, pts2d, pts3d, offsets, hypotheses, thr2, workspace, pose_out, inlier_mask, n_inliers);
-  return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+  return opb::launch_status(nullptr, __func__);
 }

@@ -11,10 +11,8 @@
 // reference network is fp32).  Everything that is not a GEMM (first layer with one input channel, 2x2 pooling, 65-way softmax
 // + pixel shuffle, NMS, ordered key-point compaction, top-k, bilinear descriptor sampling) is a plain bandwidth-bound kernel.
 #include <cmath>
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <map>
 #include <string>
 #include <vector>
 
@@ -451,10 +449,8 @@ struct SpConv {
   int cin = 0, cout = 0, bn = 0, taps = 0;
 };
 
-struct opb_superpoint {
+struct opb_superpoint : HostState {
   opb_sp_config cfg{};
-  std::string err;
-  std::map<std::string, std::vector<float>> host_w;
   bool ready = false;
   DevBuf w1a, b1a;                 // fp32 [64][9], [64]
   SpConv c1b, c2a, c2b, c3a, c3b, c4a, c4b, cPD, cPb, cDb;
@@ -462,84 +458,13 @@ struct opb_superpoint {
   int ws_B = 0, ws_H = 0, ws_W = 0;
   PlaneBuf arena[2];               // ping-pong activations
   DevBuf logits, ddesc, scores, nms, cand_idx, cand_score, blk_counts, totals;
-  int find_code = 0;               // status of the last failed weight look-up (missing: OPB_E_STATE, wrong size: OPB_E_INVALID)
   int last_B = 0, last_H = 0, last_W = 0;
-  int launches = 0;
   int stop_after = -1;             // test hook: leave the encoder after layer i (opb_sp_debug_set_stop)
   int dbg_arena = 0, dbg_c = 0;
   long long dbg_rows = 0;
-  // profiling
-  bool profiling = false;
-  std::vector<cudaEvent_t> ev;
-  std::vector<std::string> ev_name;
-  std::vector<double> ev_flops;
-  size_t ev_used = 0;
 };
 
 namespace {
-
-thread_local std::string g_sp_create_error;
-
-int sfail(opb_superpoint* h, int code, const char* fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof buf, fmt, ap);
-  va_end(ap);
-  if (h) h->err = buf; else g_sp_create_error = buf;
-  return code;
-}
-
-#define SCK(h, expr)                                                                                              \
-  do {                                                                                                            \
-    cudaError_t _e = (expr);                                                                                      \
-    if (_e != cudaSuccess)                                                                                        \
-      return sfail(h, OPB_E_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__);     \
-  } while (0)
-
-void sp_mark(opb_superpoint* h, cudaStream_t st, const char* name, double flops) {
-  h->launches++;
-  if (!h->profiling) return;
-  if (h->ev_used == h->ev.size()) {
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    h->ev.push_back(e);
-  }
-  cudaEventRecord(h->ev[h->ev_used++], st);
-  h->ev_name.push_back(name);
-  h->ev_flops.push_back(flops);
-}
-
-#define SLAUNCH(h, st, name, ...)                                                                                   \
-  do {                                                                                                              \
-    cudaError_t _le = launch_k(__VA_ARGS__);                                                                        \
-    if (_le != cudaSuccess) return sfail(h, OPB_E_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(_le));   \
-    sp_mark(h, st, name, 0.0);                                                                                      \
-  } while (0)
-
-const std::vector<float>* sp_find(opb_superpoint* h, const std::string& key, size_t n) {
-  auto it = h->host_w.find(key);
-  if (it == h->host_w.end()) { h->find_code = sfail(h, OPB_E_STATE, "missing weight '%s'", key.c_str()); return nullptr; }
-  if (it->second.size() != n) {
-    h->find_code = sfail(h, OPB_E_INVALID, "weight '%s' has %zu elements, expected %zu", key.c_str(), it->second.size(), n);
-    return nullptr;
-  }
-  return &it->second;
-}
-
-int sp_upload_planes(opb_superpoint* h, PlaneBuf& dst, const std::vector<double>& w) {
-  std::vector<__half> hi, lo;
-  split_host(w, hi, lo);
-  SCK(h, dst.ensure(w.size()));
-  SCK(h, cudaMemcpy(dst.hi.p, hi.data(), hi.size() * sizeof(__half), cudaMemcpyHostToDevice));
-  SCK(h, cudaMemcpy(dst.lo.p, lo.data(), lo.size() * sizeof(__half), cudaMemcpyHostToDevice));
-  return 0;
-}
-int sp_upload_f32(opb_superpoint* h, DevBuf& dst, const std::vector<float>& f) {
-  SCK(h, dst.ensure(f.size() * sizeof(float)));
-  SCK(h, cudaMemcpy(dst.p, f.data(), f.size() * sizeof(float), cudaMemcpyHostToDevice));
-  return 0;
-}
 
 // Pack one or two conv layers [cout, cin, k, k] (k = 3 or 1) that share their input into the B operand [cout_total (padded to
 // cout_pad), taps*cin] with reduction index tap*cin + c (tap = ky*3 + kx), plus the bias.
@@ -551,9 +476,9 @@ int sp_pack(opb_superpoint* h, SpConv& L, const std::vector<std::string>& names,
   int row0 = 0;
   for (size_t li = 0; li < names.size(); ++li) {
     const int cout = couts[li];
-    const auto* ww = sp_find(h, names[li] + ".weight", (size_t)cout * cin * taps);
-    const auto* bb = sp_find(h, names[li] + ".bias", (size_t)cout);
-    if (!ww || !bb) return h->find_code;
+    const std::vector<float> *ww, *bb;
+    if (int rc = find_w(h, names[li] + ".weight", (size_t)cout * cin * taps, ww)) return rc;
+    if (int rc = find_w(h, names[li] + ".bias", (size_t)cout, bb)) return rc;
     for (int n = 0; n < cout; ++n) {
       for (int c = 0; c < cin; ++c)
         for (int t = 0; t < taps; ++t) w[(size_t)(row0 + n) * K + (size_t)t * cin + c] = (*ww)[((size_t)n * cin + c) * taps + t];
@@ -562,8 +487,8 @@ int sp_pack(opb_superpoint* h, SpConv& L, const std::vector<std::string>& names,
     row0 += cout;
   }
   L.cin = cin; L.cout = cout_pad; L.bn = bn; L.taps = taps;
-  if (int rc = sp_upload_planes(h, L.w, w)) return rc;
-  return sp_upload_f32(h, L.b, b);
+  if (int rc = upload_planes(h, L.w, w)) return rc;
+  return upload_f32(h, L.b, b);
 }
 
 struct Stage {
@@ -583,17 +508,17 @@ int sp_ensure_workspace(opb_superpoint* h, int B, int H, int W) {
   const Stage s0 = stage_of(H, W, 0), s3 = stage_of(H, W, 3);
   const size_t elems = (size_t)Bc * s0.ppad * 64;           // the largest activation: 64 channels at full resolution
   const size_t head = (size_t)Bc * s3.ppad * 512;
-  for (int i = 0; i < 2; ++i) SCK(h, h->arena[i].ensure(elems > head ? elems : head));
-  SCK(h, h->logits.ensure((size_t)Bc * s3.ppad * 128 * sizeof(float)));
-  SCK(h, h->ddesc.ensure((size_t)Bc * s3.ppad * 256 * sizeof(float)));
+  for (int i = 0; i < 2; ++i) CK(h, h->arena[i].ensure(elems > head ? elems : head));
+  CK(h, h->logits.ensure((size_t)Bc * s3.ppad * 128 * sizeof(float)));
+  CK(h, h->ddesc.ensure((size_t)Bc * s3.ppad * 256 * sizeof(float)));
   const size_t HW = (size_t)H * W;
-  SCK(h, h->scores.ensure(Bc * HW * sizeof(float)));
-  SCK(h, h->nms.ensure(Bc * HW * sizeof(float)));
-  SCK(h, h->cand_idx.ensure(Bc * HW * sizeof(int)));
-  SCK(h, h->cand_score.ensure(Bc * HW * sizeof(float)));
-  SCK(h, h->blk_counts.ensure((size_t)Bc * ((HW + kSelChunk - 1) / kSelChunk) * sizeof(int)));
-  SCK(h, h->totals.ensure((size_t)Bc * sizeof(int)));
-  SCK(h, cudaDeviceSynchronize());
+  CK(h, h->scores.ensure(Bc * HW * sizeof(float)));
+  CK(h, h->nms.ensure(Bc * HW * sizeof(float)));
+  CK(h, h->cand_idx.ensure(Bc * HW * sizeof(int)));
+  CK(h, h->cand_score.ensure(Bc * HW * sizeof(float)));
+  CK(h, h->blk_counts.ensure((size_t)Bc * ((HW + kSelChunk - 1) / kSelChunk) * sizeof(int)));
+  CK(h, h->totals.ensure((size_t)Bc * sizeof(int)));
+  CK(h, cudaDeviceSynchronize());
   h->ws_B = Bc; h->ws_H = H; h->ws_W = W;
   return 0;
 }
@@ -625,11 +550,8 @@ int sp_run_conv(opb_superpoint* h, const SpConv& L, const PlaneBuf& in, int in_l
     p.c = outf;
     p.ldc = out_ld;
   }
-  const int rc = launch_gemm_tc(p, st);
   // algorithmic FLOPs: interior pixels only
-  sp_mark(h, st, name, 2.0 * B * g.h * g.w * (double)L.cout * L.taps * L.cin);
-  if (rc != 0) return sfail(h, rc == -1 ? OPB_E_INVALID : OPB_E_CUDA, "GEMM launch failed (%s, rc=%d): %s", name, rc, cudaGetErrorString(cudaGetLastError()));
-  return 0;
+  return run_gemm(h, p, st, 2.0 * B * g.h * g.w * (double)L.cout * L.taps * L.cin, name);
 }
 
 }  // namespace
@@ -637,48 +559,50 @@ int sp_run_conv(opb_superpoint* h, const SpConv& L, const PlaneBuf& in, int in_l
 extern "C" {
 
 int opb_sp_create(const opb_sp_config* cfg, opb_superpoint** out) {
-  if (!cfg || !out) return sfail(nullptr, OPB_E_INVALID, "null argument");
-  if (cfg->descriptor_dim != 256) return sfail(nullptr, OPB_E_INVALID, "descriptor_dim %d: only 256 is supported", cfg->descriptor_dim);
-  if (cfg->max_keypoints == 0 || cfg->max_keypoints < -1) return sfail(nullptr, OPB_E_INVALID, "\"max_keypoints\" must be positive or \"-1\"");
-  if (cfg->nms_radius < 0 || cfg->nms_radius > 6) return sfail(nullptr, OPB_E_NOT_IMPLEMENTED, "nms_radius %d: the tiled NMS supports 0..6", cfg->nms_radius);
+  if (!cfg || !out) return fail(nullptr, OPB_E_INVALID, "null argument");
+  if (cfg->descriptor_dim != 256) return fail(nullptr, OPB_E_INVALID, "descriptor_dim %d: only 256 is supported", cfg->descriptor_dim);
+  if (cfg->max_keypoints == 0 || cfg->max_keypoints < -1) return fail(nullptr, OPB_E_INVALID, "\"max_keypoints\" must be positive or \"-1\"");
+  if (cfg->nms_radius < 0 || cfg->nms_radius > 6) return fail(nullptr, OPB_E_NOT_IMPLEMENTED, "nms_radius %d: the tiled NMS supports 0..6", cfg->nms_radius);
   int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= cfg->device) return sfail(nullptr, OPB_E_CUDA, "no CUDA device %d", cfg->device);
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= cfg->device) return fail(nullptr, OPB_E_CUDA, "no CUDA device %d", cfg->device);
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, cfg->device);
-  if (prop.major != 10) return sfail(nullptr, OPB_E_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only", cfg->device, prop.major, prop.minor);
-  if (cudaSetDevice(cfg->device) != cudaSuccess) return sfail(nullptr, OPB_E_CUDA, "cudaSetDevice failed");
+  if (prop.major != 10) return fail(nullptr, OPB_E_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only", cfg->device, prop.major, prop.minor);
+  if (cudaSetDevice(cfg->device) != cudaSuccess) return fail(nullptr, OPB_E_CUDA, "cudaSetDevice failed");
   auto* h = new opb_superpoint();
   h->cfg = *cfg;
+  h->device = cfg->device;
   *out = h;
   return OPB_OK;
 }
 
 void opb_sp_destroy(opb_superpoint* h) {
   if (!h) return;
+  cudaSetDevice(h->device);
   for (SpConv* L : {&h->c1b, &h->c2a, &h->c2b, &h->c3a, &h->c3b, &h->c4a, &h->c4b, &h->cPD, &h->cPb, &h->cDb}) { L->w.release(); L->b.release(); }
   h->w1a.release(); h->b1a.release();
   h->arena[0].release(); h->arena[1].release();
   for (DevBuf* d : {&h->logits, &h->ddesc, &h->scores, &h->nms, &h->cand_idx, &h->cand_score, &h->blk_counts, &h->totals}) d->release();
-  for (auto e : h->ev) cudaEventDestroy(e);
   delete h;
 }
 
-const char* opb_sp_last_error(const opb_superpoint* h) { return h ? h->err.c_str() : g_sp_create_error.c_str(); }
+const char* opb_sp_last_error(const opb_superpoint* h) { return h ? h->err.c_str() : g_last_error.c_str(); }
 
 int opb_sp_load_weight(opb_superpoint* h, const char* name, const float* data, size_t n_elems) {
-  if (!h || !name || !data) return OPB_E_INVALID;
+  ENTER(h);
+  if (!name || !data) return fail(h, OPB_E_INVALID, "opb_sp_load_weight: null argument");
   h->host_w[name].assign(data, data + n_elems);
   h->ready = false;
   return OPB_OK;
 }
 
 int opb_sp_finalize_weights(opb_superpoint* h) {
-  if (!h) return OPB_E_INVALID;
-  const auto* w1 = sp_find(h, "conv1a.weight", 64 * 9);
-  const auto* b1 = sp_find(h, "conv1a.bias", 64);
-  if (!w1 || !b1) return h->find_code;
-  if (int rc = sp_upload_f32(h, h->w1a, *w1)) return rc;
-  if (int rc = sp_upload_f32(h, h->b1a, *b1)) return rc;
+  ENTER(h);
+  const std::vector<float> *w1, *b1;
+  if (int rc = find_w(h, "conv1a.weight", 64 * 9, w1)) return rc;
+  if (int rc = find_w(h, "conv1a.bias", 64, b1)) return rc;
+  if (int rc = upload_f32(h, h->w1a, *w1)) return rc;
+  if (int rc = upload_f32(h, h->b1a, *b1)) return rc;
   if (int rc = sp_pack(h, h->c1b, {"conv1b"}, 64, {64}, 3, 64, 64)) return rc;
   if (int rc = sp_pack(h, h->c2a, {"conv2a"}, 64, {64}, 3, 64, 64)) return rc;
   if (int rc = sp_pack(h, h->c2b, {"conv2b"}, 64, {64}, 3, 64, 64)) return rc;
@@ -691,21 +615,20 @@ int opb_sp_finalize_weights(opb_superpoint* h) {
   if (int rc = sp_pack(h, h->cPD, {"convPa", "convDa"}, 128, {256, 256}, 3, 512, 128)) return rc;
   if (int rc = sp_pack(h, h->cPb, {"convPb"}, 256, {65}, 1, 128, 128)) return rc;
   if (int rc = sp_pack(h, h->cDb, {"convDb"}, 256, {256}, 1, 256, 128)) return rc;
-  SCK(h, cudaDeviceSynchronize());
+  CK(h, cudaDeviceSynchronize());
   h->ready = true;
   return OPB_OK;
 }
 
 int opb_sp_detect(opb_superpoint* h, const float* image, int32_t B, int32_t H, int32_t W, int32_t* counts, void* stream) {
-  if (!h || !image || B <= 0 || H <= 0 || W <= 0) return h ? sfail(h, OPB_E_INVALID, "bad argument") : OPB_E_INVALID;
-  if (!h->ready) return sfail(h, OPB_E_STATE, "weights not finalized");
-  if (H % 8 || W % 8) return sfail(h, OPB_E_INVALID, "image size %dx%d: height and width must be multiples of 8 (three 2x2 poolings)", H, W);
-  if ((long long)B * stage_of(H, W, 0).ppad > 0x7fffff00LL) return sfail(h, OPB_E_INVALID, "batch too large for 32-bit row indices");
+  ENTER(h);
+  if (!image || B <= 0 || H <= 0 || W <= 0) return fail(h, OPB_E_INVALID, "bad argument");
+  if (!h->ready) return fail(h, OPB_E_STATE, "weights not finalized");
+  if (H % 8 || W % 8) return fail(h, OPB_E_INVALID, "image size %dx%d: height and width must be multiples of 8 (three 2x2 poolings)", H, W);
+  if ((long long)B * stage_of(H, W, 0).ppad > 0x7fffff00LL) return fail(h, OPB_E_INVALID, "batch too large for 32-bit row indices");
   if (int rc = sp_ensure_workspace(h, B, H, W)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  h->launches = 0;
-  h->ev_used = 0; h->ev_name.clear(); h->ev_flops.clear();
-  if (h->profiling) { sp_mark(h, st, "start", 0.0); h->launches = 0; }
+  begin_call(h, st);
   const Stage s0 = stage_of(H, W, 0), s1 = stage_of(H, W, 1), s2 = stage_of(H, W, 2), s3 = stage_of(H, W, 3);
   PlaneBuf& A = h->arena[0];
   PlaneBuf& Bf = h->arena[1];
@@ -717,27 +640,27 @@ int opb_sp_detect(opb_superpoint* h, const float* image, int32_t B, int32_t H, i
     return h->stop_after == idx;
   };
   // ---- shared encoder (superpoint.py:142-152)
-  SLAUNCH(h, st, "sp_conv1a", sp_conv1a, dim3((s0.ppad + 255) / 256, B), dim3(256), 0, st, image, (int)H, (int)W, s0.ppad, (const float*)h->w1a.as<float>(),
-          (const float*)h->b1a.as<float>(), A.hi.as<__half>(), A.lo.as<__half>());
+  LAUNCH(h, st, "sp_conv1a", sp_conv1a, dim3((s0.ppad + 255) / 256, B), dim3(256), 0, st, image, (int)H, (int)W, s0.ppad, (const float*)h->w1a.as<float>(),
+         (const float*)h->b1a.as<float>(), A.hi.as<__half>(), A.lo.as<__half>());
   if (stopped(0, 0, 64, s0)) return OPB_OK;
   if (int rc = sp_run_conv(h, h->c1b, A, 64, 0, &Bf, nullptr, 64, s0, B, 1, st, "conv1b")) return rc;
   if (stopped(1, 1, 64, s0)) return OPB_OK;
-  SLAUNCH(h, st, "sp_pool2x2", sp_pool2x2, blocks(s1.rows(B) * 8), dim3(256), 0, st, (const __half*)Bf.hi.as<__half>(), (const __half*)Bf.lo.as<__half>(), 64,
-          s0.h, s0.w, s0.ppad, A.hi.as<__half>(), A.lo.as<__half>(), s1.ppad, s1.rows(B));
+  LAUNCH(h, st, "sp_pool2x2", sp_pool2x2, blocks(s1.rows(B) * 8), dim3(256), 0, st, (const __half*)Bf.hi.as<__half>(), (const __half*)Bf.lo.as<__half>(), 64,
+         s0.h, s0.w, s0.ppad, A.hi.as<__half>(), A.lo.as<__half>(), s1.ppad, s1.rows(B));
   if (stopped(2, 0, 64, s1)) return OPB_OK;
   if (int rc = sp_run_conv(h, h->c2a, A, 64, 0, &Bf, nullptr, 64, s1, B, 1, st, "conv2a")) return rc;
   if (stopped(3, 1, 64, s1)) return OPB_OK;
   if (int rc = sp_run_conv(h, h->c2b, Bf, 64, 0, &A, nullptr, 64, s1, B, 1, st, "conv2b")) return rc;
   if (stopped(4, 0, 64, s1)) return OPB_OK;
-  SLAUNCH(h, st, "sp_pool2x2", sp_pool2x2, blocks(s2.rows(B) * 8), dim3(256), 0, st, (const __half*)A.hi.as<__half>(), (const __half*)A.lo.as<__half>(), 64,
-          s1.h, s1.w, s1.ppad, Bf.hi.as<__half>(), Bf.lo.as<__half>(), s2.ppad, s2.rows(B));
+  LAUNCH(h, st, "sp_pool2x2", sp_pool2x2, blocks(s2.rows(B) * 8), dim3(256), 0, st, (const __half*)A.hi.as<__half>(), (const __half*)A.lo.as<__half>(), 64,
+         s1.h, s1.w, s1.ppad, Bf.hi.as<__half>(), Bf.lo.as<__half>(), s2.ppad, s2.rows(B));
   if (stopped(5, 1, 64, s2)) return OPB_OK;
   if (int rc = sp_run_conv(h, h->c3a, Bf, 64, 0, &A, nullptr, 128, s2, B, 1, st, "conv3a")) return rc;
   if (stopped(6, 0, 128, s2)) return OPB_OK;
   if (int rc = sp_run_conv(h, h->c3b, A, 128, 0, &Bf, nullptr, 128, s2, B, 1, st, "conv3b")) return rc;
   if (stopped(7, 1, 128, s2)) return OPB_OK;
-  SLAUNCH(h, st, "sp_pool2x2", sp_pool2x2, blocks(s3.rows(B) * 16), dim3(256), 0, st, (const __half*)Bf.hi.as<__half>(), (const __half*)Bf.lo.as<__half>(), 128,
-          s2.h, s2.w, s2.ppad, A.hi.as<__half>(), A.lo.as<__half>(), s3.ppad, s3.rows(B));
+  LAUNCH(h, st, "sp_pool2x2", sp_pool2x2, blocks(s3.rows(B) * 16), dim3(256), 0, st, (const __half*)Bf.hi.as<__half>(), (const __half*)Bf.lo.as<__half>(), 128,
+         s2.h, s2.w, s2.ppad, A.hi.as<__half>(), A.lo.as<__half>(), s3.ppad, s3.rows(B));
   if (stopped(8, 0, 128, s3)) return OPB_OK;
   if (int rc = sp_run_conv(h, h->c4a, A, 128, 0, &Bf, nullptr, 128, s3, B, 1, st, "conv4a")) return rc;
   if (stopped(9, 1, 128, s3)) return OPB_OK;
@@ -749,41 +672,38 @@ int opb_sp_detect(opb_superpoint* h, const float* image, int32_t B, int32_t H, i
   if (int rc = sp_run_conv(h, h->cPb, Bf, 512, 0, nullptr, h->logits.as<float>(), 128, s3, B, 0, st, "convPb")) return rc;
   if (int rc = sp_run_conv(h, h->cDb, Bf, 512, 256, nullptr, h->ddesc.as<float>(), 256, s3, B, 0, st, "convDb")) return rc;
   // ---- dense scores, NMS, key-point selection (superpoint.py:157-174)
-  SLAUNCH(h, st, "sp_scores", sp_scores, blocks((long long)B * s3.h * s3.w * 32), dim3(256), 0, st, (const float*)h->logits.as<float>(), s3.h, s3.w, s3.ppad, (int)B,
-          h->scores.as<float>());
+  LAUNCH(h, st, "sp_scores", sp_scores, blocks((long long)B * s3.h * s3.w * 32), dim3(256), 0, st, (const float*)h->logits.as<float>(), s3.h, s3.w, s3.ppad, (int)B,
+         h->scores.as<float>());
   {
     const int r = h->cfg.nms_radius, D = kNmsTile + 10 * r;
     const size_t smem = (size_t)6 * D * D * sizeof(float);
-    static size_t smem_set = 0;
-    if (smem > smem_set) {
-      SCK(h, cudaFuncSetAttribute(sp_nms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      smem_set = smem;
-    }
-    SLAUNCH(h, st, "sp_nms", sp_nms, dim3((W + kNmsTile - 1) / kNmsTile, (H + kNmsTile - 1) / kNmsTile, B), dim3(512), smem, st,
-            (const float*)h->scores.as<float>(), (int)H, (int)W, r, h->nms.as<float>());
+    CK(h, ensure_smem_attr((const void*)sp_nms, (int)smem));
+    LAUNCH(h, st, "sp_nms", sp_nms, dim3((W + kNmsTile - 1) / kNmsTile, (H + kNmsTile - 1) / kNmsTile, B), dim3(512), smem, st,
+           (const float*)h->scores.as<float>(), (int)H, (int)W, r, h->nms.as<float>());
   }
   const int HW = H * W, nchunks = (HW + kSelChunk - 1) / kSelChunk;
-  SLAUNCH(h, st, "sp_count", sp_count, dim3(nchunks, B), dim3(256), 0, st, (const float*)h->nms.as<float>(), (int)H, (int)W, h->cfg.keypoint_threshold,
-          h->cfg.remove_borders, h->blk_counts.as<int>());
-  SLAUNCH(h, st, "sp_compact", sp_compact, dim3(nchunks, B), dim3(256), 0, st, (const float*)h->nms.as<float>(), (int)H, (int)W, h->cfg.keypoint_threshold,
-          h->cfg.remove_borders, (const int*)h->blk_counts.as<int>(), h->cand_idx.as<int>(), h->cand_score.as<float>(), h->totals.as<int>());
+  LAUNCH(h, st, "sp_count", sp_count, dim3(nchunks, B), dim3(256), 0, st, (const float*)h->nms.as<float>(), (int)H, (int)W, h->cfg.keypoint_threshold,
+         h->cfg.remove_borders, h->blk_counts.as<int>());
+  LAUNCH(h, st, "sp_compact", sp_compact, dim3(nchunks, B), dim3(256), 0, st, (const float*)h->nms.as<float>(), (int)H, (int)W, h->cfg.keypoint_threshold,
+         h->cfg.remove_borders, (const int*)h->blk_counts.as<int>(), h->cand_idx.as<int>(), h->cand_score.as<float>(), h->totals.as<int>());
   h->last_B = B; h->last_H = H; h->last_W = W;
   if (counts)     // number of key points opb_sp_describe will emit: min(total, max_keypoints)
-    SLAUNCH(h, st, "sp_counts_out", sp_counts_out, dim3((B + 127) / 128), dim3(128), 0, st, (const int*)h->totals.as<int>(), h->cfg.max_keypoints, (int)B, counts);
+    LAUNCH(h, st, "sp_counts_out", sp_counts_out, dim3((B + 127) / 128), dim3(128), 0, st, (const int*)h->totals.as<int>(), h->cfg.max_keypoints, (int)B, counts);
   return OPB_OK;
 }
 
 int opb_sp_describe(opb_superpoint* h, float* keypoints, float* scores, float* descriptors, int32_t* counts, int32_t cap, void* stream) {
-  if (!h || !keypoints || !scores || !counts || cap <= 0) return h ? sfail(h, OPB_E_INVALID, "bad argument") : OPB_E_INVALID;
-  if (!h->last_B) return sfail(h, OPB_E_STATE, "opb_sp_describe without a preceding opb_sp_detect");
+  ENTER(h);
+  if (!keypoints || !scores || !counts || cap <= 0) return fail(h, OPB_E_INVALID, "bad argument");
+  if (!h->last_B) return fail(h, OPB_E_STATE, "opb_sp_describe without a preceding opb_sp_detect");
   cudaStream_t st = (cudaStream_t)stream;
   const int B = h->last_B, H = h->last_H, W = h->last_W, HW = H * W;
   const Stage s3 = stage_of(H, W, 3);
-  SLAUNCH(h, st, "sp_emit", sp_emit, dim3((HW + 255) / 256, B), dim3(256), 0, st, (const int*)h->cand_idx.as<int>(), (const float*)h->cand_score.as<float>(),
-          (const int*)h->totals.as<int>(), HW, W, h->cfg.max_keypoints, (int)cap, keypoints, scores, counts);
+  LAUNCH(h, st, "sp_emit", sp_emit, dim3((HW + 255) / 256, B), dim3(256), 0, st, (const int*)h->cand_idx.as<int>(), (const float*)h->cand_score.as<float>(),
+         (const int*)h->totals.as<int>(), HW, W, h->cfg.max_keypoints, (int)cap, keypoints, scores, counts);
   if (descriptors)
-    SLAUNCH(h, st, "sp_sample", sp_sample, dim3(((long long)cap * 32 + 255) / 256, B), dim3(256), 0, st, (const float*)h->ddesc.as<float>(), s3.h, s3.w, s3.ppad,
-            (const float*)keypoints, (const int*)counts, (int)cap, h->cfg.align_corners, descriptors);
+    LAUNCH(h, st, "sp_sample", sp_sample, dim3(((long long)cap * 32 + 255) / 256, B), dim3(256), 0, st, (const float*)h->ddesc.as<float>(), s3.h, s3.w, s3.ppad,
+           (const float*)keypoints, (const int*)counts, (int)cap, h->cfg.align_corners, descriptors);
   return OPB_OK;
 }
 
@@ -796,37 +716,39 @@ int opb_sp_forward(opb_superpoint* h, const float* image, int32_t B, int32_t H, 
 int opb_sp_last_launch_count(const opb_superpoint* h) { return h ? h->launches : 0; }
 
 int opb_sp_set_profiling(opb_superpoint* h, int32_t enable) {
-  if (!h) return OPB_E_INVALID;
+  ENTER(h);
   h->profiling = enable != 0;
   return OPB_OK;
 }
 
 int opb_sp_get_profile(opb_superpoint* h, int32_t index, char* name, size_t name_cap, double* ms, double* flops) {
-  if (!h || index < 0) return OPB_E_INVALID;
-  if ((size_t)index + 1 >= h->ev_used) return OPB_E_INVALID;          // entry i = launch i (event i is the start mark)
-  cudaEventSynchronize(h->ev[index + 1]);
+  ENTER(h);
+  if (index < 0 || (size_t)index >= h->ev_name.size())                 // past the end: the caller's loop over the entries stops here
+    return fail(h, OPB_E_INVALID, "opb_sp_get_profile: no entry %d (%zu launches logged)", index, h->ev_name.size());
+  CK(h, cudaEventSynchronize(h->ev[index + 1]));
   float t = 0.f;
-  cudaEventElapsedTime(&t, h->ev[index], h->ev[index + 1]);
+  if (int rc = entry_ms(h, index, &t)) return rc;
   if (ms) *ms = t;
-  if (flops) *flops = h->ev_flops[index + 1];
-  if (name && name_cap) { strncpy(name, h->ev_name[index + 1].c_str(), name_cap - 1); name[name_cap - 1] = 0; }
+  if (flops) *flops = h->ev_flops[index];
+  if (name && name_cap) { strncpy(name, h->ev_name[index].c_str(), name_cap - 1); name[name_cap - 1] = 0; }
   return OPB_OK;
 }
 
 int opb_debug_set_conv_halo(int32_t mode) {
-  if (mode < 0 || mode > 1) return OPB_E_INVALID;
+  if (mode < 0 || mode > 1) return fail(nullptr, OPB_E_INVALID, "%s: mode %d is not 0 or 1", __func__, mode);
   set_conv_halo_mode(mode);
   return OPB_OK;
 }
 
 int opb_sp_debug_set_stop(opb_superpoint* h, int32_t layer) {
-  if (!h) return OPB_E_INVALID;
+  ENTER(h);
   h->stop_after = layer;
   return OPB_OK;
 }
 
 int opb_sp_debug_read(opb_superpoint* h, int32_t which, float* out, size_t capacity_elems, int64_t* n_elems, void* stream) {
-  if (!h || !out || !h->last_B) return OPB_E_INVALID;
+  ENTER(h);
+  if (!out || !h->last_B) return fail(h, OPB_E_INVALID, "opb_sp_debug_read: null output or no preceding opb_sp_detect");
   cudaStream_t st = (cudaStream_t)stream;
   const int B = h->last_B, H = h->last_H, W = h->last_W;
   const Stage s3 = stage_of(H, W, 3);
@@ -840,16 +762,17 @@ int opb_sp_debug_read(opb_superpoint* h, int32_t which, float* out, size_t capac
     case 4: {                                                                      // activation planes of the last layer run (stop hook)
       n = (size_t)h->dbg_rows * h->dbg_c;
       if (n_elems) *n_elems = (int64_t)n;
-      if (n > capacity_elems) return OPB_E_INVALID;
+      if (n > capacity_elems) return fail(h, OPB_E_INVALID, "opb_sp_debug_read: capacity %zu < %zu", capacity_elems, n);
       const PlaneBuf& a = h->arena[h->dbg_arena];
       sp_join_planes<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(a.hi.as<__half>(), a.lo.as<__half>(), out, (long long)n);
-      return cudaGetLastError() == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+      return launch_status(h, __func__);
     }
-    default: return OPB_E_INVALID;
+    default: return fail(h, OPB_E_INVALID, "opb_sp_debug_read: unknown buffer %d", which);
   }
   if (n_elems) *n_elems = (int64_t)n;
-  if (n > capacity_elems) return OPB_E_INVALID;
-  return cudaMemcpyAsync(out, src, n * sizeof(float), cudaMemcpyDeviceToDevice, st) == cudaSuccess ? OPB_OK : OPB_E_CUDA;
+  if (n > capacity_elems) return fail(h, OPB_E_INVALID, "opb_sp_debug_read: capacity %zu < %zu", capacity_elems, n);
+  CK(h, cudaMemcpyAsync(out, src, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return OPB_OK;
 }
 
 }  // extern "C"

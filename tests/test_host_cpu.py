@@ -160,3 +160,29 @@ def test_plain_c_client_links_and_runs(tmp_path):
     r = subprocess.run([str(exe)], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stdout + r.stderr
     assert "opb_create ->" in r.stdout and "opb_sp_create ->" in r.stdout
+
+
+def test_calls_without_a_handle_report_their_own_error():
+    """opb_last_error(NULL) is the message of this thread's last failed call without a handle: after a failed opb_create, each
+    handle-less entry point that rejects its arguments (before any CUDA work) leaves a message naming itself."""
+    import ctypes as C
+    lib = _lib.load()
+    buf = C.create_string_buffer(1024)
+    p = C.cast(buf, C.c_void_p)
+    calls = {
+        "opb_gather_features3d": lambda: lib.opb_gather_features3d(p, p, 0, 1, p, 1, p, p, 1, None),
+        "opb_segmented_mean_f64": lambda: lib.opb_segmented_mean_f64(p, p, 0, 256, p, None),
+        "opb_segmented_mean_scores_f64": lambda: lib.opb_segmented_mean_scores_f64(p, p, 0, p, None),
+        "opb_ransac_pnp": lambda: lib.opb_ransac_pnp(p, p, p, p, 0, 128, 8.0, 0, p, p, p, p, None),
+        "opb_debug_gemm": lambda: lib.opb_debug_gemm(p, p, p, p, p, 1, 256, 64, 0, None),
+        "opb_forward": lambda: lib.opb_forward(None, p, None, 1, 1, p, p, p, p, p, None),
+    }
+    for name, call in calls.items():
+        bad = _lib.OpbConfig(128, 4, 0.07, 0.2, 1, 0, 0, 0)          # rejected before any CUDA call
+        h = C.c_void_p()
+        assert lib.opb_create(C.byref(bad), C.byref(h)) == -1
+        assert b"descriptor_dim" in lib.opb_last_error(None)
+        assert call() == -1, name
+        msg = lib.opb_last_error(None)
+        assert name.encode() in msg and b"descriptor_dim" not in msg, (name, msg)
+        assert lib.opb_sp_last_error(None) == msg                    # one slot for both handle types
